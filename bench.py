@@ -21,6 +21,14 @@ N > 1   ONE planning problem on all ranks: the same nominal policy everywhere, N
              with the reference's own thread rule (nproc - 3) and the fp32 instantiation beside it.
 
 --impl reference times that CPU path as its own arm.
+
+Inputs: the nominal comes from a burn-in on the fp64 CPU oracle and the candidate noise from seeded Philox counters,
+so the same arguments give the same inputs bit for bit, whichever build of the engine runs.
+--dump-outputs DIR writes what the last timed step returned (DIR/<name>.npy, float32 / float64): the headline
+launch's returns, failure flags, ranking and every candidate trajectory, and the end-to-end call's returns, failure
+flags, ranking and winner trajectory (prefix e2e_).  Two builds are compared output for output on these files.
+
+The bench runs on the library that build() left in the tree and writes nothing into the tree.
 """
 from __future__ import annotations
 
@@ -31,6 +39,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True   # the tree may be read-only: no __pycache__ from the imports below
 
 import numpy as np
 
@@ -322,6 +332,21 @@ def hbm_peak():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_LIMIT = 64 << 20   # bytes, all --dump-outputs files together
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy; flags and indices are stored as float64 (exact)."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_reference(args, rank, world):
     """--impl reference: the CPU port of the path (the reference binary cannot be built offline: MuJoCo is fetched at
     configure time) on all usable host cores, its own burn-in, bounded sample."""
@@ -359,7 +384,10 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-probes", action="store_true", help="skip the iLQG / Humanoid Track probes (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", 0)); local = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -373,12 +401,7 @@ def main():
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    from mujoco_mpc_b200 import build
     from mujoco_mpc_b200.engine import Engine
-    if rank == 0:
-        build.build()
-    if world > 1:
-        dist.barrier()
     n_iter = args.steps + args.warmup
     from conftest import get_model
     n_total = world * N_CAND                                   # one problem: N x 256 candidates
@@ -387,8 +410,10 @@ def main():
     eng = Engine(get_model("quadruped"), N_CAND, HORIZON, device=local)
     if world > 1:
         eng.comm_init_torch(dist)                              # ncclCommInitRank inside libmjpc_b200.so
-    # the burn-in runs on this rank's GPU alone with 256 candidates: deterministic, so every rank holds the same nominal
-    m, state, mocap, knots, kt, nominal_return = load_inputs(eng, n_iter, n_cand=n_total)
+    # the burn-in runs on the fp64 CPU oracle with 256 candidates (its result does not depend on the thread count):
+    # every rank, and every build of the engine, gets the same nominal
+    burn_in = OracleBackend(get_model("quadruped"), max(1, usable_cores() // world))
+    m, state, mocap, knots, kt, nominal_return = load_inputs(burn_in, n_iter, n_cand=n_total)
     P = knots[0].shape[1]
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device="cuda")  # > 126 MB L2
 
@@ -422,7 +447,7 @@ def main():
             eng.launch_resident()
             eng.sync()
         else:
-            eng.rollout_spline_sharded(state, 0.0, mocap, knots[it], kt, INTERP, HORIZON)
+            sharded_out = eng.rollout_spline_sharded(state, 0.0, mocap, knots[it], kt, INTERP, HORIZON)
         if it >= args.warmup:
             kern_ms.append(eng.last_kernel_ms)
     barrier()
@@ -430,6 +455,12 @@ def main():
     gpu_launches = eng.launch_count - launches0
     ms_per_step = max_over_ranks(float(np.sum(kern_ms))) / args.steps
     value = n_total * HORIZON / (ms_per_step * 1e-3)
+    outputs = {}
+    if args.dump_outputs and rank == 0:      # read back after the timed region: what the last timed step computed
+        ret, fail, order = eng.read_returns() if world == 1 else sharded_out
+        outputs.update(returns=ret, failure=fail, order=order)
+        if world == 1:
+            outputs.update(eng.fetch_all())
 
     # ---------------- end-to-end through the public call with host buffers (collective included at N > 1)
     ds, nu, nr, ntr = eng.ds, eng.nu, eng.nr, eng.ntr
@@ -443,15 +474,17 @@ def main():
         else:
             ret, fail, order = eng.rollout_spline_sharded(state, 0.0, mocap, knots[it], kt, INTERP, HORIZON)
             best = eng.fetch_trajectory_sharded(int(order[0]))     # ncclBroadcast from the winner's owner
-        return ret, order, best
+        return ret, fail, order, best
     for it in range(args.warmup):
         e2e_step(it)
     barrier()
     t0 = time.perf_counter()
     for it in range(args.steps):
-        ret, order, best = e2e_step(args.warmup + it)
+        ret, fail, order, best = e2e_step(args.warmup + it)
     barrier()
     e2e_value = n_total * HORIZON / max_over_ranks((time.perf_counter() - t0) / args.steps)
+    if args.dump_outputs and rank == 0:
+        outputs.update(e2e_returns=ret, e2e_failure=fail, e2e_order=order, **{"e2e_winner_" + k: v for k, v in best.items()})
     clk = clocks.stop()      # samples cover both timed regions (device-timed and end-to-end), 50 ms apart
 
     # ---------------- N > 1: one-problem evidence + strong scaling of the 256-candidate problem
@@ -573,7 +606,7 @@ def main():
             "data": "synthetic",
             "config": {"workload": WORKLOAD if world == 1 else WORKLOAD + "; N GPUs: one planning problem, %d candidates sharded %d per GPU" % (n_total, N_CAND),
                        "model": model_fidelity(m), "candidates_per_gpu": N_CAND, "candidates_total": n_total, "horizon": HORIZON, "spline_points": P,
-                       "nominal": "steady-state policy after %d planning iterations from the zero policy (return %.4f)" % (BURN_IN, nominal_return),
+                       "nominal": "steady-state policy after %d planning iterations of the fp64 CPU oracle from the zero policy (return %.4f)" % (BURN_IN, nominal_return),
                        "l2": "flushed between timed iterations (256 MB memset)",
                        "sharding": "one problem, contiguous candidate ranges, one ncclAllGather of returns per iteration" if world > 1 else "single GPU",
                        "e2e_call": ("Engine.rollout_spline (mjpc_b200_rollout_spline) + fetch_trajectory(winner), host buffers" if world == 1 else
@@ -582,6 +615,8 @@ def main():
             "clocks": clk, "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
             "gpu_launches": int(gpu_launches), "roofline": roofline, "cpu_baseline": cpu, "parity": parity, "ilqg": ilqg, "humanoid_track": config3, "shadow_reorient_standin": config5,
             "multi_gpu": multi, "wall_s_timed_region": wall}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
