@@ -105,6 +105,24 @@ int mjpc_b200_rollout_spline(mjpc_b200_t* h, const float* state, double time, co
                              const float* userdata, const float* knots, const double* knot_times, int interp,
                              int P, int N, int H, float* returns, uint8_t* failure, int* order);
 
+/* Per-problem task snapshot of a batched rollout; a NULL member = the handle's current value for every problem. */
+typedef struct {
+  const double* weight;      /* [M][num_term]                                                             */
+  const double* parameters;  /* [M][num_parameters]                                                       */
+  const double* task_state;  /* [M][task_state_size] (absolute times; rebased per problem like set_task's) */
+} mjpc_task_batch;
+
+/* M independent planning problems of this handle's model in ONE launch: problem p is (state [p], time [p], mocap [p],
+ * task rows p, knots [p][N][P][nu], knot_times [p][P]); all share N, P, H, interp and the handle's risk, timestep,
+ * differentiable flag and xfrc noise settings.  Problem p's returns [p][N], failure [p][N] and order [p][N] (problem-local
+ * indices, ascending return, ties: lower index first; may be NULL) are bit for bit what mjpc_b200_rollout_spline returns
+ * for that problem alone, and so are its trajectories: fetch_trajectory / fetch_all / fetch_stats see the M*N candidates
+ * problem-major (candidate i of problem p is p*N + i).  M*N above max_candidates returns MJPC_B200_ERR_CAPACITY; mocap
+ * [M][7 nmocap] is required when nmocap > 0; userdata is not accepted.  Never uses a communicator (comm_init). */
+int mjpc_b200_rollout_spline_batched(mjpc_b200_t* h, int M, const float* state, const double* time, const float* mocap,
+                                     const mjpc_task_batch* task, const float* knots, const double* knot_times, int interp,
+                                     int P, int N, int H, float* returns, uint8_t* failure, int* order);
+
 /* NoisyRollout (mjpc/trajectory.cc:100-210, used by the Robust planner): the following rollouts of this handle add
  * Ornstein-Uhlenbeck noise to xfrc_applied of every body (stationary std xfrc_std, correlation time xfrc_rate
  * seconds), drawn from Philox4x32-10 with key (seed, 1) and counter (step, candidate, element, 'XFRC') - the
@@ -236,6 +254,26 @@ int mjpc_b200_planner_optimize_policy(void* planner, int horizon);          /* S
 void mjpc_b200_planner_action_from_policy(void* planner, double* action, double time, int use_previous);
 int mjpc_b200_planner_get_result(void* planner, int* winner, double* improvement, float* returns, double* knots,
                                  double* knot_times);
+
+/* ---- Batched Predictive Sampling (csrc/host/batch_sampling_planner.{h,cc}): num_agents independent SamplingPlanners
+ * (agent p seeded with seeds[p]) on ONE engine handle.  Every agent has its own policy, previous policy, iteration
+ * counter, state, time, mocap and task snapshot (initially the model's; set_task's NULL members keep the agent's value,
+ * its risk applies to all agents).  optimize_policy makes each agent's candidates as the single planner does, rolls all
+ * of them out with ONE mjpc_b200_rollout_spline_batched launch and installs each agent's winner: agent p's results are
+ * bit for bit those of a single planner with seed seeds[p] and the same inputs.  The per-agent calls take an agent index
+ * in [0, num_agents). */
+int mjpc_b200_batch_planner_create(const mjpc_model_blob* model, int num_agents, const uint32_t* seeds, int num_trajectory,
+                                   int num_spline_points, int interpolation, double exploration, double timestep,
+                                   const double* ctrlrange, int max_horizon, int device, void** out);
+void mjpc_b200_batch_planner_destroy(void* planner);
+void mjpc_b200_batch_planner_reset(void* planner, int agent, int horizon, const double* initial_repeated_action);
+void mjpc_b200_batch_planner_set_state(void* planner, int agent, const double* state, double time, const double* mocap);
+int mjpc_b200_batch_planner_set_task(void* planner, int agent, const mjpc_task_desc* task);
+int mjpc_b200_batch_planner_optimize_policy(void* planner, int horizon);    /* all agents, one launch; 0 or -1 */
+void mjpc_b200_batch_planner_action_from_policy(void* planner, int agent, double* action, double time, int use_previous);
+/* as mjpc_b200_planner_get_result, for one agent */
+int mjpc_b200_batch_planner_get_result(void* planner, int agent, int* winner, double* improvement, float* returns,
+                                       double* knots, double* knot_times);
 
 /* ---- Cross-Entropy planner (csrc/host/cross_entropy_planner.{h,cc}; mjpc/planners/cross_entropy/planner.h:35-146).
  * One rollout launch covers the N noisy candidates and the un-noised nominal (candidate N); the elite mean and

@@ -31,6 +31,7 @@ def needs_build():
 def _compile(verbose):
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
     cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", SO, os.path.join(CSRC, "engine.cu"), os.path.join(CSRC, "host", "sampling_planner.cc"),
+                                                                           os.path.join(CSRC, "host", "batch_sampling_planner.cc"),
                                                                            os.path.join(CSRC, "host", "cross_entropy_planner.cc"),
                                                                            os.path.join(CSRC, "host", "ilqg_planner.cc"),
                                                                            os.path.join(CSRC, "host", "robust_planner.cc"),

@@ -91,6 +91,12 @@ struct mjpc_b200 {
   int maxTotal = 0;
   int nuserdata = 0;
   int differentiable = 0;   // MakeDifferentiable (utilities.cc:60-75) for the following launches (DevModel::differentiable)
+  // batched rollouts (mjpc_b200_rollout_spline_batched): per-problem rows for up to max_candidates problems, packed per
+  // call as [state | mocap | task_state | weight | parameters | knot_times] and uploaded with one copy; knots use d_knots
+  float* d_batch = nullptr;
+  double* d_time0s = nullptr;
+  float* h_batch = nullptr;
+  double* h_time0s = nullptr;
   // resident-input launch description
   RolloutArgs resident;
   bool resident_ok = false;
@@ -145,9 +151,12 @@ Staged stage_common(mjpc_b200* h, const float* state, double time, const float* 
 
 int launch_rollout(mjpc_b200* h, const RolloutArgs& A_in) {
   RolloutArgs A = A_in;
+  // A.nprob > 0: the batched instances, A.nprob problems of A.N candidates; a CTA never holds two problems' candidates
+  const bool batched = A.nprob > 0;
+  const int nprob = batched ? A.nprob : 1, total = nprob * A.N;
   const int wpc = h->warps_per_cta;
   const size_t smem = h->smem_bytes(A.P, wpc);
-  const int grid = (A.N + wpc - 1) / wpc;
+  const int grid = nprob * ((A.N + wpc - 1) / wpc);
   CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
   // static instance: same arguments, same shared-memory image; MJPC_B200_NO_STATIC=1 forces the generic kernel
   const char* ns = std::getenv("MJPC_B200_NO_STATIC");
@@ -156,7 +165,7 @@ int launch_rollout(mjpc_b200* h, const RolloutArgs& A_in) {
   // at once (one wave); MJPC_B200_PAIR_SYNC=0 switches it off (profiling)
   {
     const char* ps = std::getenv("MJPC_B200_PAIR_SYNC");
-    const bool on = !(ps && ps[0] == '0') && A.N > h->num_sms && A.N <= 2 * h->num_sms;
+    const bool on = !(ps && ps[0] == '0') && total > h->num_sms && total <= 2 * h->num_sms;
     A.pair_sync = on ? h->d_pair_sync : nullptr;
     A.pair_sync_mode = (ps && ps[0] >= '1' && ps[0] <= '9') ? std::atoi(ps) : 1;   // 1: meet per step (default), 3: and before the solve; + 16 k: only at steps with (t & k) == 0
     if (on) CUDA_TRY(cudaMemsetAsync(h->d_pair_sync, 0, (size_t)256 * 32 * sizeof(unsigned), h->stream));
@@ -165,20 +174,27 @@ int launch_rollout(mjpc_b200* h, const RolloutArgs& A_in) {
   const char* sh = std::getenv("MJPC_B200_SHAPE");
   const bool plain = sh && sh[0] == 'p' && sh[1] == 'l';
   if (use_static && h->static_spec == 1) {
-    if (plain) rollout_kernel_quadruped_plain<<<grid, 32, smem, h->stream>>>(A);
+    if (batched && plain) rollout_kernel_quadruped_plain_batched<<<grid, 32, smem, h->stream>>>(A);
+    else if (batched) rollout_kernel_quadruped_batched<<<grid, kRolloutThreads, smem, h->stream>>>(A);
+    else if (plain) rollout_kernel_quadruped_plain<<<grid, 32, smem, h->stream>>>(A);
     else rollout_kernel_quadruped<<<grid, kRolloutThreads, smem, h->stream>>>(A);
   } else if (use_static && h->static_spec == 2) {
-    if (plain) rollout_kernel_humanoid_track_plain<<<grid, 32, smem, h->stream>>>(A);
+    if (batched && plain) rollout_kernel_humanoid_track_plain_batched<<<grid, 32, smem, h->stream>>>(A);
+    else if (batched) rollout_kernel_humanoid_track_batched<<<grid, kRolloutThreads, smem, h->stream>>>(A);
+    else if (plain) rollout_kernel_humanoid_track_plain<<<grid, 32, smem, h->stream>>>(A);
     else rollout_kernel_humanoid_track<<<grid, kRolloutThreads, smem, h->stream>>>(A);
+  } else if (batched) {
+    rollout_kernel_batched<<<grid, 32 * wpc, smem, h->stream>>>(A);
   } else {
     rollout_kernel<<<grid, 32 * wpc, smem, h->stream>>>(A);
   }
   h->last_static = use_static ? (plain ? 2 : 1) : 0;
-  rank_kernel<<<(A.N + 255) / 256, 256, 0, h->stream>>>(A.returns, A.N, h->d_order);
+  if (batched) rank_batched_kernel<<<(total + 255) / 256, 256, 0, h->stream>>>(A.returns, nprob, A.N, h->d_order);
+  else rank_kernel<<<(A.N + 255) / 256, 256, 0, h->stream>>>(A.returns, A.N, h->d_order);
   CUDA_TRY(cudaEventRecord(h->ev1, h->stream));
   CUDA_TRY(cudaGetLastError());
   h->launches += 2;
-  h->lastN = A.N; h->lastH = A.H;
+  h->lastN = total; h->lastH = A.H;
   return 0;
 }
 
@@ -358,16 +374,26 @@ int mjpc_b200_create(const mjpc_model_blob* model, int max_candidates, int max_h
   CREATE_TRY(cudaMallocHost((void**)&h->h_in, h->h_in_floats * 4));
   h->h_out_bytes = N * 16 + 64;
   CREATE_TRY(cudaMallocHost((void**)&h->h_out, h->h_out_bytes));
+  {
+    const size_t row = ds + 7 * (size_t)M.nmocap + M.task_state_size + M.num_term + M.num_parameters + h->maxP;
+    CREATE_TRY(dalloc(&h->d_batch, N * row)); CREATE_TRY(dalloc(&h->d_time0s, N));
+    CREATE_TRY(cudaMallocHost((void**)&h->h_batch, N * row * 4)); CREATE_TRY(cudaMallocHost((void**)&h->h_time0s, N * 8));
+  }
   if (int rc = set_smem((const void*)rollout_kernel, h->smem_bytes(h->maxP, h->warps_per_cta))) { mjpc_b200_destroy(h); return rc; }
+  if (int rc = set_smem((const void*)rollout_kernel_batched, h->smem_bytes(h->maxP, h->warps_per_cta))) { mjpc_b200_destroy(h); return rc; }
   if (int rc = set_smem((const void*)step_debug_kernel, h->smem_bytes(1, 1))) { mjpc_b200_destroy(h); return rc; }
   if (spec_matches<SpecQuadruped>(M, make_layout(M, 1))) {
     h->static_spec = 1;
     if (int rc = set_smem((const void*)rollout_kernel_quadruped, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
     if (int rc = set_smem((const void*)rollout_kernel_quadruped_plain, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
+    if (int rc = set_smem((const void*)rollout_kernel_quadruped_batched, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
+    if (int rc = set_smem((const void*)rollout_kernel_quadruped_plain_batched, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
   } else if (spec_matches<SpecHumanoidTrack>(M, make_layout(M, 1))) {
     h->static_spec = 2;
     if (int rc = set_smem((const void*)rollout_kernel_humanoid_track, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
     if (int rc = set_smem((const void*)rollout_kernel_humanoid_track_plain, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
+    if (int rc = set_smem((const void*)rollout_kernel_humanoid_track_batched, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
+    if (int rc = set_smem((const void*)rollout_kernel_humanoid_track_plain_batched, h->smem_bytes(h->maxP, 1))) { mjpc_b200_destroy(h); return rc; }
   }
   if (int rc = ilqg_init(h->ilqg, h->pack.M, (int)H, h->smem_bytes(1, 1))) {
     mjpc_b200_destroy(h);
@@ -386,11 +412,14 @@ void mjpc_b200_destroy(mjpc_b200_t* h) {
   for (void* p : mbufs) if (p) cudaFree(p);
   void* bufs[] = {h->d_pack, h->d_state, h->d_mocap, h->d_task_state, h->d_knots, h->d_knot_times, h->d_unom, h->d_xnom,
                   h->d_tnom, h->d_gains, h->d_du, h->d_steps, h->d_states, h->d_actions, h->d_times, h->d_residual,
-                  h->d_costs, h->d_trace, h->d_returns, h->d_failure, h->d_order, h->d_dbg, h->d_stats, h->d_pair_sync};
+                  h->d_costs, h->d_trace, h->d_returns, h->d_failure, h->d_order, h->d_dbg, h->d_stats, h->d_pair_sync,
+                  h->d_batch, h->d_time0s};
   for (void* p : bufs) if (p) cudaFree(p);
   ilqg_free(h->ilqg);
   if (h->h_in) cudaFreeHost(h->h_in);
   if (h->h_out) cudaFreeHost(h->h_out);
+  if (h->h_batch) cudaFreeHost(h->h_batch);
+  if (h->h_time0s) cudaFreeHost(h->h_time0s);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -498,6 +527,58 @@ int mjpc_b200_rollout_spline(mjpc_b200_t* h, const float* state, double time, co
   rc = launch_rollout(h, h->resident);
   if (rc) return rc;
   return read_back(h, N, returns, failure, order);
+}
+
+// M independent problems of the same model in one launch.  Every per-problem input is converted exactly as
+// upload_spline_inputs / upload_task convert a single problem's (knot and task-state times rebased to the problem's own
+// start, weights and parameters rounded to float), so problem p computes bit for bit what rollout_spline computes for it.
+int mjpc_b200_rollout_spline_batched(mjpc_b200_t* h, int M, const float* state, const double* time, const float* mocap,
+                                     const mjpc_task_batch* task, const float* knots, const double* knot_times, int interp,
+                                     int P, int N, int H, float* returns, uint8_t* failure, int* order) {
+  if (!h || !state || !time || !knots || !knot_times) return fail(MJPC_B200_ERR_BAD_ARGUMENT, "rollout_spline_batched: null pointer");
+  const DevModel& D = h->pack.M;
+  if (D.nmocap && !mocap) return fail(MJPC_B200_ERR_BAD_ARGUMENT, "rollout_spline_batched: mocap required");
+  if (M < 1 || N < 1 || H < 1 || P < 1 || interp < 0 || interp > 2)
+    return fail(MJPC_B200_ERR_BAD_ARGUMENT, "rollout_spline_batched: bad sizes");
+  if ((int64_t)M * N > h->maxN || H > h->maxH || P > h->maxP)
+    return fail(MJPC_B200_ERR_CAPACITY, "rollout_spline_batched: M*N/H/P above capacity");
+  CUDA_TRY(cudaSetDevice(h->device));
+  const size_t ds = D.nq + D.nv, nm = 7 * (size_t)D.nmocap, nts = D.task_state_size, nw = D.num_term,
+               np = D.num_parameters, nk = (size_t)N * P * D.nu;
+  const size_t o_state = 0, o_mocap = o_state + M * ds, o_ts = o_mocap + M * nm, o_w = o_ts + M * nts, o_p = o_w + M * nw,
+               o_kt = o_p + M * np, end = o_kt + (size_t)M * P;
+  float* b = h->h_batch;
+  std::memcpy(b + o_state, state, M * ds * 4);
+  if (nm) std::memcpy(b + o_mocap, mocap, M * nm * 4);
+  const double* tw = task ? task->weight : nullptr;
+  const double* tp = task ? task->parameters : nullptr;
+  const double* tts = task ? task->task_state : nullptr;
+  for (int p = 0; p < M; p++) {
+    const double t0 = time[p];
+    h->h_time0s[p] = t0;
+    for (size_t i = 0; i < nts; i++) {
+      double v = tts ? tts[p * nts + i] : h->task_state[i];
+      if (std::find(h->time_idx.begin(), h->time_idx.end(), (int)i) != h->time_idx.end()) v -= t0;
+      b[o_ts + p * nts + i] = (float)v;
+    }
+    for (size_t i = 0; i < nw; i++) b[o_w + p * nw + i] = (float)(tw ? tw[p * nw + i] : h->weight[i]);
+    for (size_t i = 0; i < np; i++) b[o_p + p * np + i] = (float)(tp ? tp[p * np + i] : h->parameters[i]);
+    for (int k = 0; k < P; k++) b[o_kt + (size_t)p * P + k] = (float)(knot_times[(size_t)p * P + k] - t0);
+  }
+  std::memcpy(h->h_in, knots, M * nk * 4);
+  CUDA_TRY(cudaMemcpyAsync(h->d_batch, b, end * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_TRY(cudaMemcpyAsync(h->d_time0s, h->h_time0s, (size_t)M * 8, cudaMemcpyHostToDevice, h->stream));
+  CUDA_TRY(cudaMemcpyAsync(h->d_knots, h->h_in, M * nk * 4, cudaMemcpyHostToDevice, h->stream));
+  RolloutArgs A = base_args(h, time[0], N, H);
+  A.L = make_layout(h->pack.M, P);
+  A.state = h->d_batch + o_state; A.mocap = h->d_batch + o_mocap; A.task_state = h->d_batch + o_ts;
+  A.task_weight = h->d_batch + o_w; A.task_parameters = h->d_batch + o_p;
+  A.knots = h->d_knots; A.knot_times = h->d_batch + o_kt; A.P = P; A.interp = interp; A.policy_kind = 0;
+  A.nprob = M; A.time0s = h->d_time0s;
+  h->resident_ok = false;   // d_knots now holds the batch
+  int rc = launch_rollout(h, A);
+  if (rc) return rc;
+  return read_back(h, M * N, returns, failure, order);
 }
 
 int mjpc_b200_rollout_feedback(mjpc_b200_t* h, const float* state, double time, const float* mocap,

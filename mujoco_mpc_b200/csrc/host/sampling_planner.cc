@@ -84,7 +84,17 @@ int SamplingPlanner::Initialize(const mjpc_model_blob* model, int num_trajectory
                                 uint32_t seed, int max_candidates, int max_horizon, int device) {
   int rc = mjpc_b200_create(model, max_candidates, max_horizon, device, &gpu_);
   if (rc) return rc;
-  mjpc_b200_get_info(gpu_, &info_);
+  mjpc_b200_info info;
+  mjpc_b200_get_info(gpu_, &info);
+  InitializeHost(info, num_trajectory, num_spline_points, interpolation, exploration, exploration2, timestep, ctrlrange, seed,
+                 max_candidates);
+  return 0;
+}
+
+void SamplingPlanner::InitializeHost(const mjpc_b200_info& info, int num_trajectory, int num_spline_points, int interpolation,
+                                     double exploration, double exploration2, double timestep, const double* ctrlrange,
+                                     uint32_t seed, int max_candidates) {
+  info_ = info;
   nu_ = info_.nu;
   num_trajectory_ = num_trajectory;
   interpolation_ = (SplineInterpolation)interpolation;
@@ -98,7 +108,6 @@ int SamplingPlanner::Initialize(const mjpc_model_blob* model, int num_trajectory
   state_.assign(info_.dim_state, 0.0); mocap_.assign(7 * info_.nmocap, 0.0);
   returns_.assign(max_candidates, 0.f); failure_.assign(max_candidates, 0);
   winner = 0;
-  return 0;
 }
 
 void SamplingPlanner::Reset(int, const double* initial_repeated_action) {
@@ -155,7 +164,7 @@ void SamplingPlanner::AddNoiseToPolicy(int i) {
   }
 }
 
-int SamplingPlanner::Rollouts(int num_trajectory, int horizon) {
+void SamplingPlanner::MakeCandidates(int num_trajectory) {
   const int P = policy.plan.Size();
   knots_.resize((size_t)num_trajectory * P * nu_);
   knot_times_.resize(P);
@@ -171,6 +180,11 @@ int SamplingPlanner::Rollouts(int num_trajectory, int horizon) {
     }
   }
   for (int k = 0; k < P; k++) knot_times_[k] = policy.plan.NodeTime(k);
+}
+
+int SamplingPlanner::Rollouts(int num_trajectory, int horizon) {
+  MakeCandidates(num_trajectory);
+  const int P = policy.plan.Size();
   std::vector<float> state_f(state_.begin(), state_.end()), mocap_f(mocap_.begin(), mocap_.end());
   trajectory_order.resize(num_trajectory);
   return mjpc_b200_rollout_spline(gpu_, state_f.data(), time_, mocap_f.empty() ? nullptr : mocap_f.data(), nullptr,
@@ -189,11 +203,15 @@ int SamplingPlanner::OptimizePolicyCandidates(int ncandidates, int horizon) {
 
 int SamplingPlanner::OptimizePolicy(int horizon) {
   if (OptimizePolicyCandidates(1, horizon) < 0) return -1;
+  InstallWinner();
+  return 0;
+}
+
+void SamplingPlanner::InstallWinner() {
   CopyCandidateToPolicy(0);
   const double best_return = returns_[0];   // candidate 0 is the un-noised nominal
   improvement = std::max(best_return - (double)returns_[winner], 0.0);
   iteration++;
-  return 0;
 }
 
 void SamplingPlanner::CopyCandidateToPolicy(int candidate) {

@@ -63,13 +63,19 @@ class SamplingPlanner {
   int Initialize(const mjpc_model_blob* model, int num_trajectory, int num_spline_points, int interpolation,
                  double exploration, double exploration2, double timestep, const double* ctrlrange, uint32_t seed,
                  int max_candidates, int max_horizon, int device);
+  // the same without an engine handle: a planner whose rollouts another object launches (BatchSamplingPlanner)
+  void InitializeHost(const mjpc_b200_info& info, int num_trajectory, int num_spline_points, int interpolation,
+                      double exploration, double exploration2, double timestep, const double* ctrlrange, uint32_t seed,
+                      int max_candidates);
   void Reset(int horizon, const double* initial_repeated_action);
   void SetState(const double* state, double time, const double* mocap);
   int OptimizePolicy(int horizon);                    // planner.cc:197-212
   int OptimizePolicyCandidates(int ncandidates, int horizon);   // :155-194
   void UpdateNominalPolicy(int horizon);              // :240-323 (non-sliding resample)
   void AddNoiseToPolicy(int i);                       // :326-352
-  int Rollouts(int num_trajectory, int horizon);      // :355-393 -> one C-ABI call
+  int Rollouts(int num_trajectory, int horizon);      // :355-393 -> MakeCandidates + one C-ABI call
+  void MakeCandidates(int num_trajectory);            // candidate policies (nominal + noise) and their knots
+  void InstallWinner();                               // OptimizePolicy after the rollouts: best candidate -> policy
   void ActionFromPolicy(double* action, double time, bool use_previous = false);   // :229-237
   void CopyCandidateToPolicy(int candidate);          // :534-543
   const Trajectory* BestTrajectory();
@@ -93,6 +99,7 @@ class SamplingPlanner {
   void SetExploration(double e0, double e1) { noise_exploration_[0] = e0; noise_exploration_[1] = e1; }
 
  private:
+  friend class BatchSamplingPlanner;                  // launches the rollouts of many planners at once
   mjpc_b200_t* gpu_ = nullptr;
   mjpc_b200_info info_{};
   int num_trajectory_ = 0, nu_ = 0;

@@ -4,6 +4,8 @@
 //                       (Trajectory::Rollout / RolloutDiscrete,
 //                       mjpc/trajectory.cc:92-309) incl. policy, mj_step restatement, residual, cost, return
 //   rank_kernel         order of candidates by return (partial_sort, sampling/planner.cc:184-188)
+//   *_batched           the rollout instances for M independent problems in one launch (rollout_body<SP, true>),
+//   rank_batched_kernel   ranked per problem (DESIGN.md section 6a)
 //   step_debug_kernel   a single forward+Euler step through the same device functions (parity hook)
 //   fd_*_kernel         finite-difference transition/residual Jacobians (model_derivatives.cc:45-165)
 //
@@ -40,6 +42,12 @@ struct RolloutArgs {
   int pair_sync_mode;       // bit 0: meet at every time step, bit 1: also before every constraint solve
   unsigned* pair_sync;      // HBM [256][32] zeroed before the launch, or nullptr: co-resident pair synchronisation (dev_data.cuh)
   long long* stats;         // [N][12]: cycles, Newton iterations, contacts, constraint rows (summed over steps), 8 phase timers
+  // batched instances only (rollout_body<SP, true>): `nprob` problems of N candidates each, candidate p*N + i of the launch
+  // is candidate i of problem p; state, mocap, task_state and knot_times above then hold one row per problem
+  int nprob;
+  const double* time0s;          // [nprob] absolute start time of each problem
+  const float* task_weight;      // [nprob][num_term]
+  const float* task_parameters;  // [nprob][num_parameters]
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -159,16 +167,29 @@ __device__ __noinline__ void task_warp_loop(Ctx& c, const RolloutArgs& A, int ca
   }
 }
 
-template <class SP>
+// kBatch: A.nprob independent problems in one launch.  A CTA never spans two problems (the grid holds ceil(N / candidates
+// per CTA) CTAs per problem), so the per-CTA shared-memory copies of the task weights, parameters and state can be
+// overwritten with the problem's rows before the task warp forks.  Outputs are indexed by the launch-wide candidate p*N + i;
+// the xfrc noise stream uses the problem-local index i, so every problem computes what a launch of that problem alone does.
+template <class SP, bool kBatch = false>
 __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
   float* smem = g_smem;
   stage_model_pack(smem, A.pack, (unsigned)((A.M.nf + A.M.ni) * 4));
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // SP::kWide > 1: the whole CTA is ONE candidate (warp 0 runs the pipeline, the others help with the wide phases)
-  const int cand = (SP::kWide > 1 || SP::kTask > 0) ? (int)blockIdx.x : blockIdx.x * (blockDim.x >> 5) + warp;
+  constexpr bool kCtaPerCand = SP::kWide > 1 || SP::kTask > 0;
+  int cand = kCtaPerCand ? (int)blockIdx.x : blockIdx.x * (blockDim.x >> 5) + warp;
+  int prob = 0, local = cand;   // problem and problem-local candidate (batched instances)
+  if constexpr (kBatch) {
+    const int per_cta = kCtaPerCand ? 1 : (int)(blockDim.x >> 5);
+    const int ctas = (A.N + per_cta - 1) / per_cta;   // CTAs per problem
+    prob = (int)blockIdx.x / ctas;
+    local = ((int)blockIdx.x - prob * ctas) * per_cta + (kCtaPerCand ? 0 : warp);
+    cand = prob * A.N + local;
+  }
   Ctx c;
-  init_ctx(c, &A.M, &A.L, smem, (SP::kWide > 1 || SP::kTask > 0) ? 0 : warp, lane, A.pack);
-  if (cand >= A.N) return;
+  init_ctx(c, &A.M, &A.L, smem, kCtaPerCand ? 0 : warp, lane, A.pack);
+  if (local >= A.N) return;
   if (SP::kWide > 1 && warp > 0 && warp < SP::kWide) { wide_helper_loop<SP>(c); return; }
   if (SP::kTask > 0 && warp == SP::kWide) { task_warp_loop<SP>(c, A, cand); return; }
   constexpr bool kTask = SP::kTask > 0;
@@ -176,18 +197,27 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
   if constexpr (SP::kWide > 1) pair_sync_init(c, A.pair_sync, A.pair_sync_mode);
   auto&& M = SP::model(c);
   const int nq = M.nq, nv = M.nv, nu = M.nu, ds = nq + nv, nr = M.num_residual, ntr = 3 * M.num_trace, H = A.H;
+  // this problem's row of a per-problem input (the single-problem instances read the argument itself at every use)
+#define ROW(field, width) (kBatch ? A.field + (size_t)prob * (width) : A.field)
+#define TIME0 (kBatch ? A.time0s[prob] : A.time0)
   // per-iteration task state (time-rebased) overrides the packed copy: the pack in shared memory is per CTA,
   // every warp writes the same values
   if (A.task_state) {
     float* ts = const_cast<float*>(MF(task_state));
-    for (int i = lane; i < M.task_state_size; i += 32) ts[i] = A.task_state[i];
+    for (int i = lane; i < M.task_state_size; i += 32) ts[i] = ROW(task_state, M.task_state_size)[i];
+  }
+  if constexpr (kBatch) {   // ... and so do the problem's task weights and parameters
+    float* w = const_cast<float*>(MF(task_weight));
+    float* prm = const_cast<float*>(MF(task_parameters));
+    for (int i = lane; i < M.num_term; i += 32) w[i] = A.task_weight[(size_t)prob * M.num_term + i];
+    for (int i = lane; i < M.num_parameters; i += 32) prm[i] = A.task_parameters[(size_t)prob * M.num_parameters + i];
   }
   // ---- initial conditions (trajectory.cc:108-137)
-  for (int i = lane; i < nq; i += 32) DF(qpos)[i] = A.state[i];
-  for (int i = lane; i < nv; i += 32) { DF(qvel)[i] = A.state[nq + i]; DF(qacc_warmstart)[i] = 0; }
+  for (int i = lane; i < nq; i += 32) DF(qpos)[i] = ROW(state, ds)[i];
+  for (int i = lane; i < nv; i += 32) { DF(qvel)[i] = ROW(state, ds)[nq + i]; DF(qacc_warmstart)[i] = 0; }
   for (int i = lane; i < 7 * M.nmocap; i += 32) {
     const int k = i / 7, q = i - 7 * k;
-    if (q < 3) DF(mocap_pos)[3 * k + q] = A.mocap[i]; else DF(mocap_quat)[4 * k + q - 3] = A.mocap[i];
+    if (q < 3) DF(mocap_pos)[3 * k + q] = ROW(mocap, 7 * M.nmocap)[i]; else DF(mocap_quat)[4 * k + q - 3] = ROW(mocap, 7 * M.nmocap)[i];
   }
   for (int i = lane; i < nv * nv; i += 32) DF(qM)[i] = 0;
   const bool noisy = A.xfrc_std > 0.f;
@@ -198,7 +228,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
   float step_size = 0.f;
   if (A.policy_kind == 0) {
     for (int i = lane; i < A.P * nu; i += 32) DF(knots)[i] = A.knots[(size_t)cand * A.P * nu + i];
-    for (int i = lane; i < A.P; i += 32) DF(knot_times)[i] = A.knot_times[i];
+    for (int i = lane; i < A.P; i += 32) DF(knot_times)[i] = ROW(knot_times, A.P)[i];
   } else {
     step_size = A.step_sizes[cand];
   }
@@ -209,8 +239,8 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
   float* o_res = A.residual + (size_t)cand * H * nr;
   float* o_costs = A.costs + (size_t)cand * H;
   float* o_trace = A.trace + (size_t)cand * H * ntr;
-  for (int i = lane; i < ds; i += 32) o_states[i] = A.state[i];
-  if (lane == 0) o_times[0] = A.time0;
+  for (int i = lane; i < ds; i += 32) o_states[i] = ROW(state, ds)[i];
+  if (lane == 0) o_times[0] = TIME0;
   float total = 0.f;
   bool failed = false;
   const long long clk0 = clock64();
@@ -236,7 +266,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
     if (noisy && !last) {   // Ornstein-Uhlenbeck perturbation in discrete time (trajectory.cc:147-155)
       float* xf = DF(xfrc);
       for (int i = lane; i < 6 * M.nbody; i += 32)
-        xf[i] = ou_rate * xf[i] + ou_scale * xfrc_normal(A.noise_seed, (unsigned)t, (unsigned)(A.cand0 + cand), (unsigned)i);
+        xf[i] = ou_rate * xf[i] + ou_scale * xfrc_normal(A.noise_seed, (unsigned)t, (unsigned)(A.cand0 + local), (unsigned)i);
       __syncwarp();
     }
     float cost;
@@ -285,7 +315,7 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
     k_euler<SP>(c);
     for (int i = lane; i < nq; i += 32) o_states[(size_t)(t + 1) * ds + i] = DF(qpos)[i];
     for (int i = lane; i < nv; i += 32) o_states[(size_t)(t + 1) * ds + nq + i] = DF(qvel)[i];
-    if (lane == 0) o_times[t + 1] = A.time0 + (double)c.time;
+    if (lane == 0) o_times[t + 1] = TIME0 + (double)c.time;
   }
   pair_sync_done(c);
   wide_post<SP>(c, WIDE_EXIT);   // releases the helper warps
@@ -311,6 +341,8 @@ __device__ __forceinline__ void rollout_body(const RolloutArgs& A) {
 #endif
     }
   }
+#undef ROW
+#undef TIME0
 }
 
 extern "C" __global__ void __launch_bounds__(128) rollout_kernel(const __grid_constant__ RolloutArgs A) {
@@ -341,6 +373,25 @@ extern "C" __global__ void __launch_bounds__(kRolloutThreads) rollout_kernel_hum
 extern "C" __global__ void __launch_bounds__(32) rollout_kernel_humanoid_track_plain(const __grid_constant__ RolloutArgs A) {
   rollout_body<StaticSpec<SpecHumanoidTrack, 1, 0>>(A);
 }
+// Batched twins of the five instances above: A.nprob problems of A.N candidates in one launch (rollout_body<SP, true>).
+// Batched<SP> is SP under another name, so the batched kernels get their own copies of the SP-templated non-inlined
+// device functions and leave the register allocation of the single-problem kernels' copies exactly as it was.
+template <class SP> struct Batched : SP {};
+extern "C" __global__ void __launch_bounds__(128) rollout_kernel_batched(const __grid_constant__ RolloutArgs A) {
+  rollout_body<Batched<DynSpec>, true>(A);
+}
+extern "C" __global__ void __launch_bounds__(kRolloutThreads) rollout_kernel_quadruped_batched(const __grid_constant__ RolloutArgs A) {
+  rollout_body<Batched<StaticSpec<SpecQuadruped, kRolloutWide, kRolloutTask>>, true>(A);
+}
+extern "C" __global__ void __launch_bounds__(32) rollout_kernel_quadruped_plain_batched(const __grid_constant__ RolloutArgs A) {
+  rollout_body<Batched<StaticSpec<SpecQuadruped, 1, 0>>, true>(A);
+}
+extern "C" __global__ void __launch_bounds__(kRolloutThreads) rollout_kernel_humanoid_track_batched(const __grid_constant__ RolloutArgs A) {
+  rollout_body<Batched<StaticSpec<SpecHumanoidTrack, kRolloutWide, kRolloutTask>>, true>(A);
+}
+extern "C" __global__ void __launch_bounds__(32) rollout_kernel_humanoid_track_plain_batched(const __grid_constant__ RolloutArgs A) {
+  rollout_body<Batched<StaticSpec<SpecHumanoidTrack, 1, 0>>, true>(A);
+}
 
 // host: does the live model header / state layout equal the table a static kernel was compiled from?
 // (float options are not part of the comparison: static kernels read them from the live header)
@@ -367,6 +418,21 @@ extern "C" __global__ void rank_kernel(const float* __restrict__ ret, int N, int
       rank += (rj < ri) || (rj == ri && j < i) || (ri != ri && rj == rj);
     }
     order[rank] = i;
+  }
+}
+
+// the same per problem: ret [M][N] -> order [M][N] of problem-local indices (rank_kernel's comparison, NaN last)
+extern "C" __global__ void rank_batched_kernel(const float* __restrict__ ret, int M, int N, int* __restrict__ order) {
+  for (int g = blockIdx.x * blockDim.x + threadIdx.x; g < M * N; g += gridDim.x * blockDim.x) {
+    const int p = g / N, i = g - p * N;
+    const float* r = ret + (size_t)p * N;
+    const float ri = r[i];
+    int rank = 0;
+    for (int j = 0; j < N; j++) {
+      const float rj = r[j];
+      rank += (rj < ri) || (rj == ri && j < i) || (ri != ri && rj == rj);
+    }
+    order[(size_t)p * N + rank] = i;
   }
 }
 

@@ -19,7 +19,7 @@ _ip = C.POINTER(C.c_int)
 _bp = C.POINTER(C.c_uint8)
 
 EXPORTS = ["mjpc_b200_version", "mjpc_b200_last_error", "mjpc_b200_create", "mjpc_b200_destroy",
-           "mjpc_b200_get_info", "mjpc_b200_set_task", "mjpc_b200_set_differentiable", "mjpc_b200_set_xfrc_noise", "mjpc_b200_rollout_spline", "mjpc_b200_rollout_feedback",
+           "mjpc_b200_get_info", "mjpc_b200_set_task", "mjpc_b200_set_differentiable", "mjpc_b200_set_xfrc_noise", "mjpc_b200_rollout_spline", "mjpc_b200_rollout_spline_batched", "mjpc_b200_rollout_feedback",
            "mjpc_b200_fetch_trajectory", "mjpc_b200_fetch_all", "mjpc_b200_model_derivatives",
            "mjpc_b200_cost_derivatives", "mjpc_b200_backward_pass", "mjpc_b200_step_debug", "mjpc_b200_step_batch", "mjpc_b200_comm_unique_id", "mjpc_b200_comm_init",
            "mjpc_b200_comm_info", "mjpc_b200_rollout_spline_sharded", "mjpc_b200_fetch_trajectory_sharded",
@@ -30,6 +30,9 @@ EXPORTS = ["mjpc_b200_version", "mjpc_b200_last_error", "mjpc_b200_create", "mjp
            "mjpc_b200_planner_create", "mjpc_b200_planner_destroy", "mjpc_b200_planner_set_exploration", "mjpc_b200_planner_reset",
            "mjpc_b200_planner_set_state", "mjpc_b200_planner_optimize_policy",
            "mjpc_b200_planner_action_from_policy", "mjpc_b200_planner_get_result",
+           "mjpc_b200_batch_planner_create", "mjpc_b200_batch_planner_destroy", "mjpc_b200_batch_planner_reset",
+           "mjpc_b200_batch_planner_set_state", "mjpc_b200_batch_planner_set_task", "mjpc_b200_batch_planner_optimize_policy",
+           "mjpc_b200_batch_planner_action_from_policy", "mjpc_b200_batch_planner_get_result",
            "mjpc_b200_ce_planner_create", "mjpc_b200_ce_planner_destroy", "mjpc_b200_ce_planner_reset",
            "mjpc_b200_ce_planner_set_state", "mjpc_b200_ce_planner_optimize_policy",
            "mjpc_b200_ce_planner_action_from_policy", "mjpc_b200_ce_planner_get_result",
@@ -65,6 +68,10 @@ class TaskDesc(C.Structure):
     _fields_ = [("weight", _dp), ("parameters", _dp), ("task_state", _dp), ("risk", C.c_double)]
 
 
+class TaskBatch(C.Structure):
+    _fields_ = [("weight", _dp), ("parameters", _dp), ("task_state", _dp)]
+
+
 class Info(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("nq", "nv", "nu", "na", "nmocap", "nuserdata", "dim_state", "dim_dstate",
                                        "num_residual", "num_term", "num_trace", "num_parameters", "task_state_size",
@@ -90,6 +97,7 @@ def load_library():
         lib.mjpc_b200_planner_destroy.argtypes = [C.c_void_p]
         lib.mjpc_b200_planner_set_exploration.argtypes = [C.c_void_p, C.c_double, C.c_double]
         lib.mjpc_b200_ce_planner_destroy.argtypes = [C.c_void_p]
+        lib.mjpc_b200_batch_planner_destroy.argtypes = [C.c_void_p]
         lib.mjpc_b200_ilqg_planner_destroy.argtypes = [C.c_void_p]
         for n in ("mjpc_b200_ilqg_planner_set_fd", "mjpc_b200_gradient_planner_set_fd", "mjpc_b200_ilqs_planner_set_fd"):
             getattr(lib, n).argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_int]
@@ -149,6 +157,32 @@ def _pd(a):
     return None if a is None else a.ctypes.data_as(_dp)
 
 
+def batched_inputs(m, state, time, mocap, knots, knot_times, weight=None, parameters=None, task_state=None):
+    """The arguments of Engine.rollout_spline_batched for model m as contiguous arrays of the C ABI's types; raises
+    ValueError when a shape does not fit knots [M][N][P][nu]."""
+    knots = _f(knots)
+    if knots.ndim != 4 or knots.shape[3] != m.nu or min(knots.shape) < 1:
+        raise ValueError(f"knots must be [M][N][P][{m.nu}], got {knots.shape}")
+    M, N, P, _ = knots.shape
+
+    def rows(a, width, conv, name, optional=False):
+        if a is None:
+            if optional:
+                return None
+            raise ValueError(f"{name} is required")
+        a = conv(a)
+        if a.shape != (M, width):
+            raise ValueError(f"{name} must be [{M}][{width}], got {a.shape}")
+        return a
+    tm = _d(time)
+    if tm.shape != (M,):
+        raise ValueError(f"time must be [{M}], got {tm.shape}")
+    return (rows(state, m.nq + m.nv, _f, "state"), tm, rows(mocap, 7 * m.nmocap, _f, "mocap") if m.nmocap else None,
+            knots, rows(knot_times, P, _d, "knot_times"), rows(weight, len(m.task_weight), _d, "weight", True),
+            rows(parameters, len(m.task_parameters), _d, "parameters", True),
+            rows(task_state, len(m.task_state), _d, "task_state", True))
+
+
 class Engine:
     """One handle = one GPU's share of the candidates (Planner::Initialize/Allocate analogue)."""
 
@@ -205,6 +239,23 @@ class Engine:
                                                       _pd(kt), int(interp), P, N, int(H), _pf(ret),
                                                       fail.ctypes.data_as(_bp), order.ctypes.data_as(_ip)))
         self.lastN, self.lastH = N, H
+        return ret, fail, order
+
+    def rollout_spline_batched(self, state, time, mocap, knots, knot_times, interp, H, weight=None, parameters=None,
+                               task_state=None):
+        """M independent problems in one launch (mjpc_b200_rollout_spline_batched): state [M][dim_state], time [M],
+        mocap [M][7 nmocap], knots [M][N][P][nu], knot_times [M][P] (absolute), optional task rows [M][...] (None = the
+        handle's current value for every problem).  Returns returns [M][N], failure [M][N], order [M][N] (problem-local)."""
+        st, tm, mc, knots, kt, w, p, ts = batched_inputs(self.m, state, time, mocap, knots, knot_times, weight, parameters,
+                                                         task_state)
+        M, N, P, _ = knots.shape
+        task = TaskBatch(_pd(w), _pd(p), _pd(ts)) if any(a is not None for a in (w, p, ts)) else None
+        ret = np.zeros((M, N), np.float32); fail = np.zeros((M, N), np.uint8); order = np.zeros((M, N), np.int32)
+        self._check(self.lib.mjpc_b200_rollout_spline_batched(self.h, M, _pf(st), _pd(tm), _pf(mc),
+                                                              C.byref(task) if task is not None else None, _pf(knots),
+                                                              _pd(kt), int(interp), P, N, int(H), _pf(ret),
+                                                              fail.ctypes.data_as(_bp), order.ctypes.data_as(_ip)))
+        self.lastN, self.lastH = M * N, H
         return ret, fail, order
 
     # ---- multi-GPU: one planning problem sharded over an NCCL communicator owned by the handle
@@ -455,6 +506,79 @@ class CppSamplingPlanner:
     def action_from_policy(self, time, use_previous=False):
         a = np.zeros(self.nu)
         self.lib.mjpc_b200_planner_action_from_policy(self.h, _pd(a), C.c_double(time), int(use_previous))
+        return a
+
+
+class BatchSamplingPlanner:
+    """The C++ batched Predictive Sampling planner (csrc/host/batch_sampling_planner.cc): num_agents independent agents,
+    agent p seeded with seeds[p], every iteration ONE batched launch on one engine handle."""
+
+    def __init__(self, model, num_agents, num_trajectory, horizon, seeds=None, device=0):
+        self.lib = load_library()
+        m = self.m = model
+        self._blob = to_blob(model)
+        self._buf = C.create_string_buffer(self._blob, len(self._blob))
+        mb = ModelBlob(C.cast(self._buf, C.c_void_p), len(self._blob))
+        num = m.numeric
+        self.P = int(num.get("sampling_spline_points", [3])[0])
+        self.M, self.horizon, self.N, self.nu = int(num_agents), int(horizon), int(num_trajectory), m.nu
+        sd = np.ascontiguousarray([0x5EED] * self.M if seeds is None else seeds, np.uint32)
+        if sd.shape != (self.M,):
+            raise ValueError(f"seeds must have {self.M} entries")
+        cr = _d(np.asarray(m.actuator_ctrlrange, float).reshape(-1))
+        h = C.c_void_p()
+        rc = self.lib.mjpc_b200_batch_planner_create(
+            C.byref(mb), self.M, sd.ctypes.data_as(C.POINTER(C.c_uint32)), self.N, self.P,
+            int(num.get("sampling_representation", [2])[0]), C.c_double(float(num.get("sampling_exploration", [0.1])[0])),
+            C.c_double(float(m.opt_timestep)), _pd(cr), self.horizon, int(device), C.byref(h))
+        if rc != 0:
+            raise EngineError(f"mjpc_b200_batch_planner_create failed ({rc}): {self.lib.mjpc_b200_last_error().decode()}")
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.lib.mjpc_b200_batch_planner_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def _agent(self, agent):
+        if not 0 <= int(agent) < self.M:
+            raise IndexError(f"agent {agent} outside [0, {self.M})")
+        return int(agent)
+
+    def reset(self, agent, initial_repeated_action=None):
+        a = _d(initial_repeated_action)
+        self.lib.mjpc_b200_batch_planner_reset(self.h, self._agent(agent), self.horizon, _pd(a))
+
+    def set_state(self, agent, state, time, mocap):
+        s, mc = _d(state), _d(mocap)
+        self.lib.mjpc_b200_batch_planner_set_state(self.h, self._agent(agent), _pd(s), C.c_double(time), _pd(mc))
+
+    def set_task(self, agent, weight=None, parameters=None, task_state=None, risk=None):
+        w, p, s = _d(weight), _d(parameters), _d(task_state)
+        td = TaskDesc(_pd(w), _pd(p), _pd(s), float(self.m.task_risk if risk is None else risk))
+        rc = self.lib.mjpc_b200_batch_planner_set_task(self.h, self._agent(agent), C.byref(td))
+        if rc != 0:
+            raise EngineError(f"batch_planner_set_task failed ({rc}): {self.lib.mjpc_b200_last_error().decode()}")
+
+    def optimize_policy(self):
+        rc = self.lib.mjpc_b200_batch_planner_optimize_policy(self.h, self.horizon)
+        if rc != 0:
+            raise EngineError(f"batch_planner_optimize_policy failed: {self.lib.mjpc_b200_last_error().decode()}")
+        return [self.result(p) for p in range(self.M)]
+
+    def result(self, agent):
+        winner, imp = C.c_int(), C.c_double()
+        ret = np.zeros(self.N, np.float32); knots = np.zeros((self.P, self.nu)); kt = np.zeros(self.P)
+        self.lib.mjpc_b200_batch_planner_get_result(self.h, self._agent(agent), C.byref(winner), C.byref(imp), _pf(ret),
+                                                    _pd(knots), _pd(kt))
+        return dict(winner=winner.value, improvement=imp.value, returns=ret, knots=knots, knot_times=kt)
+
+    def action_from_policy(self, agent, time, use_previous=False):
+        a = np.zeros(self.nu)
+        self.lib.mjpc_b200_batch_planner_action_from_policy(self.h, self._agent(agent), _pd(a), C.c_double(time),
+                                                            int(use_previous))
         return a
 
 

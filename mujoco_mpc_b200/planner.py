@@ -144,15 +144,81 @@ class SamplingPlanner:
         knots = self.make_candidates()
         ret, fail, order = self.backend.rollout_spline(self.state, self.time, self.mocap, knots, self.times,
                                                        self.interp, self.horizon)
+        self.install_winner(knots, ret, order)
+        return ret, fail
+
+    def install_winner(self, knots, ret, order):
+        """The rest of OptimizePolicy once the candidates are rolled out: the best one becomes the policy."""
         self.winner = int(order[0]) if order is not None else int(np.argmin(ret))
         self.improvement = max(float(ret[0]) - float(ret[self.winner]), 0.0)
         self.values = knots[self.winner].astype(float)
         self.returns = ret
         self.iteration += 1
-        return ret, fail
 
     def action_from_policy(self, time):
         return clamp(sample_spline(self.times, self.values, self.interp, time), self.ctrlrange)
+
+
+_TASK_ATTR = dict(weight="task_weight", parameters="task_parameters", task_state="task_state")   # model attributes
+
+
+class BatchSamplingPlanner:
+    """M independent Predictive Sampling agents of one model, planned together (csrc/host/batch_sampling_planner.cc).
+
+    Each agent is a SamplingPlanner (own policy, seed, iteration, state, time, mocap) with its own task snapshot.  Per
+    optimize_policy every agent makes its candidates, then ONE backend.rollout_spline_batched call rolls all of them out
+    when the backend has it; otherwise (the CPU oracle) backend.rollout_spline runs per agent, after backend.set_task with
+    that agent's snapshot when any agent has one.  Snapshot members an agent never set are the model's values."""
+
+    def __init__(self, model, backend, num_agents, num_trajectory=None, horizon=None, seeds=None):
+        self.model, self.backend, self.M = model, backend, int(num_agents)
+        seeds = [0x5EED] * self.M if seeds is None else list(seeds)
+        if len(seeds) != self.M:
+            raise ValueError(f"seeds must have {self.M} entries")
+        self.agents = [SamplingPlanner(model, backend, num_trajectory, horizon, sd) for sd in seeds]
+        self.tasks = [dict() for _ in range(self.M)]
+
+    def reset(self, agent, initial_repeated_action=None):
+        self.agents[agent].reset(initial_repeated_action)
+
+    def set_state(self, agent, state, time, mocap):
+        self.agents[agent].set_state(state, time, mocap)
+
+    def set_task(self, agent, weight=None, parameters=None, task_state=None):
+        for k, v in (("weight", weight), ("parameters", parameters), ("task_state", task_state)):
+            if v is not None:
+                self.tasks[agent][k] = np.array(v, float)
+
+    def _task_rows(self, key):
+        """[M][...] rows of one snapshot member, or None when no agent set it."""
+        if not any(key in t for t in self.tasks):
+            return None
+        default = np.asarray(getattr(self.model, _TASK_ATTR[key]), float)
+        return np.stack([t.get(key, default) for t in self.tasks])
+
+    def optimize_policy(self):
+        a0 = self.agents[0]
+        knots = np.stack([a.make_candidates() for a in self.agents])
+        rows = {k: self._task_rows(k) for k in ("weight", "parameters", "task_state")}
+        if hasattr(self.backend, "rollout_spline_batched"):
+            ret, fail, order = self.backend.rollout_spline_batched(
+                np.stack([a.state for a in self.agents]), np.array([a.time for a in self.agents]),
+                np.stack([a.mocap for a in self.agents]), knots, np.stack([a.times for a in self.agents]), a0.interp,
+                a0.horizon, **rows)
+        else:
+            ret, fail, order = [], [], []
+            for p, a in enumerate(self.agents):
+                if any(r is not None for r in rows.values()):
+                    self.backend.set_task(**{k: (getattr(self.model, _TASK_ATTR[k]) if r is None else r[p])
+                                             for k, r in rows.items()})
+                r, f, o = self.backend.rollout_spline(a.state, a.time, a.mocap, knots[p], a.times, a.interp, a.horizon)
+                ret.append(r); fail.append(f); order.append(o)
+        for p, a in enumerate(self.agents):
+            a.install_winner(knots[p], ret[p], order[p])
+        return np.asarray(ret), np.asarray(fail)
+
+    def action_from_policy(self, agent, time):
+        return self.agents[agent].action_from_policy(time)
 
 
 class CrossEntropyPlanner:

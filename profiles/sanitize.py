@@ -37,4 +37,16 @@ if which in ("all", "humanoid"):
     eh.rollout_spline(sh, 0.0, mc, kh, np.arange(16) * 0.003, 2, 8)
     del os.environ["MJPC_B200_NO_STATIC"]
     g = eh.step_debug(mh.qpos0, np.zeros(mh.nv), np.zeros(mh.nu), mc)
+if which in ("all", "batched"):                                                # batched instances: 2 problems x 3 candidates
+    M2 = 2
+    args = (np.tile(state, (M2, 1)), np.arange(M2) * 0.1, np.tile(mocap, (M2, 1)), np.stack([knots[:3]] * M2),
+            np.stack([kt + 0.1 * p for p in range(M2)]), 2, 10)
+    for shape in ("wide", "plain"):
+        os.environ["MJPC_B200_SHAPE"] = shape
+        e.rollout_spline_batched(*args)
+        assert e.last_kernel_shape == (1 if shape == "wide" else 2)
+    del os.environ["MJPC_B200_SHAPE"]
+    os.environ["MJPC_B200_NO_STATIC"] = "1"
+    e.rollout_spline_batched(*args)                                            # generic instance
+    del os.environ["MJPC_B200_NO_STATIC"]
 print("sanitize run done:", which)
